@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200-native Open-DiffusionGS hot path.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--dump-outputs DIR]
   (N > 1: launched by the driver as  python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...)
 
 Metric (BASELINE.json): denoise-steps/s (+ rasterized-views/s) at 256x256.
@@ -17,6 +17,8 @@ gradient all-reduce and again without any, and adds `train: [{samples_per_s, ms_
 Prints ONE JSON line (rank 0).  Keys: the driver contract + `roofline` (dominant kernel, live CUDA-event
 timing through the library's per-family event hooks) + `cpu_baseline` (oracle on the host cores, bounded
 sample) + `e2e` (same metric through the public API with pinned-host inputs, H2D/D2H inside the timed region).
+`--dump-outputs DIR` writes what the last timed step returned (the rendered views and the Gaussians) as DIR/<name>.npy in
+float32, so that two builds can be compared output for output on the same seeded inputs.
 `--impl reference` times the reference's CPU path = the oracle port (the reference has no CPU rasterizer and
 its Python package does not import offline; see DESIGN.md) on the host cores.
 """
@@ -43,6 +45,8 @@ LAYERS = 24
 D = 1024
 N_TOK = 2 + V * (H // PATCH) * (W // PATCH)
 P_GAUSS = 2 + V * H * W
+GAUSSIAN_FIELDS = ("xyz", "features", "scaling", "rotation", "opacity")
+DUMP_BYTES = 64 << 20
 
 
 def dit_forward_flops(n_tok=N_TOK, layers=LAYERS, d=D):
@@ -97,6 +101,20 @@ def make_batch(batch, seed):
     t = np.full((batch,), 500, np.int64)
     tt = torch.from_numpy
     return dict(image=tt(image), ray_o=tt(ray_o), ray_d=tt(ray_d), c2w=tt(c2w), fxfycxcy=tt(fx), t=tt(t))
+
+
+def dump_outputs(out_dir, arrays, cap=DUMP_BYTES, seed=0):
+    """Writes every tensor of `arrays` as out_dir/<name>.npy in float32.  If they come to more than `cap` bytes, every
+    array keeps the same fraction of its entries, chosen by a fixed seed (flattened, in index order), so that runs with
+    the same arguments write comparable files."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    frac = min(1.0, cap / sum(4 * a.numel() for a in arrays.values()))
+    for name, a in arrays.items():
+        a = a.detach().float().cpu().numpy()
+        if frac < 1.0:
+            a = a.ravel()[np.sort(np.random.default_rng(seed).choice(a.size, int(a.size * frac), replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -439,7 +457,13 @@ def main():
     ap.add_argument("--no-overlap", action="store_true", help="train workload: all-reduce after the whole backward")
     ap.add_argument("--train-batches", default="4,8", help="per-GPU batch sizes of the training section (N > 1)")
     ap.add_argument("--no-train-section", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (rendered views, Gaussians) as DIR/<name>.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "denoise"):
+        ap.error("--dump-outputs applies to the denoise workload of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -475,8 +499,13 @@ def main():
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)  # > 126 MB L2
     L = _lib.lib()
 
-    def step(b):
+    keep = bool(args.dump_outputs)
+    last_gaussians = {}
+
+    def step(b, keep=False):
         params, _ = model.image_to_gaussians(b["image"], b["ray_o"], b["ray_d"], b["t"])
+        if keep:
+            last_gaussians.update((k, params[k]) for k in GAUSSIAN_FIELDS)
         return model.render_gaussians(params, b["c2w"], b["fxfycxcy"], H, W)
 
     def barrier():
@@ -488,12 +517,12 @@ def main():
     sampler = ClockSampler(local_rank)  # every rank samples its own GPU (per-rank clocks / power in the N > 1 line);
     sampler.start()                     # started BEFORE the warm-up: spawning nvidia-smi right before the timed region cost the first timed step 5 ms (r2, N = 2)
     for _ in range(args.warmup):
-        img = step(devb)
+        img = step(devb, keep)  # with --dump-outputs the timed steps keep their Gaussians alive; so do these
     # N > 1: the clocks / power of a box that just went from idle to N busy GPUs settle over the first ~100 ms (r1 SCALE:
     # the first timed region was slower than the later wall-timed e2e loop); extra UNTIMED steps, same on every rank
     for _ in range(30 if world > 1 else 0):
         flush.zero_()
-        img = step(devb)
+        img = step(devb, keep)
     barrier()
 
     # ---- timed region 1: inputs resident in HBM, per-step CUDA events, L2 flushed between steps ----
@@ -505,10 +534,12 @@ def main():
     for a, b_ in ev:
         flush.zero_()
         a.record()
-        img = step(devb)
+        img = step(devb, keep)
         b_.record()
     barrier()
     t_wall1 = time.time()
+    # the last timed step's outputs are tensors of their own (not workspace), so the later regions do not overwrite them
+    last_outputs = dict(render=img, **last_gaussians) if keep else None
     launches = L.dgs_kernel_launch_count() - launches0
     clocks = sampler.stop(t_wall0, t_wall1)
     step_ms = [a.elapsed_time(b_) for a, b_ in ev]
@@ -582,6 +613,8 @@ def main():
         dist.destroy_process_group()
     if rank != 0:
         return
+    if last_outputs is not None:
+        dump_outputs(args.dump_outputs, last_outputs)
 
     # ---- roofline of the dominant kernel family ----
     peaks = load_peaks()

@@ -5,6 +5,9 @@ executed by path from /root/reference on CPU tensors.  Only the compiled `_C` ex
 oracle (oracle/raster.py, itself held to the reference's CUDA kernels by tests/golden/ref_*.npz).  Stored: the seeded
 inputs, the rendered views and the five parameter gradients of a seeded cotangent.
 
+Also writes tests/golden/gaussian_model_ref.npz: what the reference's GaussianModel (gs_core.py:386-475, 578-633) keeps
+after apply_all_filters on seeded Gaussians, and the PLY property list it builds.
+
     python tests/golden/make_renderer_golden.py        # needs /root/reference (this container)
 """
 import os
@@ -24,6 +27,10 @@ NAMES = ("xyz", "features", "scaling", "rotation", "opacity")
 # name -> (B, V, P, W, H, distribution, seed)
 CASES = {"trained_b2v3": (2, 3, 1500, 64, 48, "trained", 0), "init_b1v2": (1, 2, 800, 48, 48, "init", 5),
          "fine_b1v4": (1, 4, 3000, 80, 64, "fine", 9)}
+GAUSSIAN_MODEL = os.path.join(HERE, "gaussian_model_ref.npz")
+GAUSSIAN_MODEL_FIELDS = ("_xyz", "_features_dc", "_scaling", "_rotation", "_opacity")
+FILTERS = dict(opacity_thres=0.05, crop_bbx=[-1, 1, -1, 1, -1, 1],
+               cam_origins=torch.tensor([[0.0, 0.0, 3.0], [3.0, 0.0, 0.0], [0.0, 3.0, 1.0]]), nearfar_percent=(0.005, 1.0))
 
 
 def inputs(case):
@@ -51,7 +58,24 @@ def run_reference(case):
     return raw, c2w, fx, dimg, img.detach().numpy(), {k: p.grad.numpy() for k, p in zip(NAMES, params)}
 
 
+def gaussian_data(n=500, seed=0):
+    """(xyz, features, scaling, rotation, opacity) of n seeded Gaussians, SH degree 0"""
+    g = torch.Generator().manual_seed(seed)
+    return (torch.randn(n, 3, generator=g) * 0.8, torch.randn(n, 1, 3, generator=g), torch.randn(n, 3, generator=g) - 3,
+            torch.randn(n, 4, generator=g), torch.randn(n, 1, generator=g) * 2)
+
+
+def write_gaussian_model():
+    ref = ri.load("oracle").gs_core.GaussianModel(0).set_data(*gaussian_data())
+    ref.apply_all_filters(**FILTERS)
+    rec = {k: getattr(ref, k).numpy() for k in GAUSSIAN_MODEL_FIELDS}
+    rec["dtypes"] = np.array([f"{n}:{t}" for n, t in ref.construct_dtypes()])
+    np.savez_compressed(GAUSSIAN_MODEL, **rec)
+    print(GAUSSIAN_MODEL, os.path.getsize(GAUSSIAN_MODEL), "bytes")
+
+
 def main():
+    write_gaussian_model()
     for case in CASES:
         raw, c2w, fx, dimg, img, grads = run_reference(case)
         rec = {"in/" + k: v for k, v in raw.items()}

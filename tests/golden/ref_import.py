@@ -292,10 +292,14 @@ def seeded_state_dict(module, seed):
     stable): matrices ~ N(0, 1/fan_in) so activations stay O(1) through the depth, biases / adaLN biases ~ N(0, 0.1^2)
     (the reference's zero-initialised biases would leave those code paths untested), LayerNorm weights 1 + N(0, 0.1^2),
     the Gaussian position embedding ~ N(0, 1)."""
+    return seeded_params({k: tuple(v.shape) for k, v in module.state_dict().items()}, seed)
+
+
+def seeded_params(shapes, seed):
+    """seeded_state_dict for an ordered {name: shape}; the values depend on the order of the names."""
     rng = np.random.default_rng(seed)
     sd = {}
-    for k, v in module.state_dict().items():
-        shape = tuple(v.shape)
+    for k, shape in shapes.items():
         if k.endswith("layernorm.weight"):
             a = 1.0 + 0.1 * rng.standard_normal(shape)
         elif k.endswith(".bias"):
@@ -331,6 +335,23 @@ DIT_CASES = {
     "w1024_obj_plk": (False, "plk", dict(width=1024, dim_heads=64, num_layers=2, patch_size=8), (1, 2, 32, 32), 23),
 }
 GS_KEYS = ("xyz", "features", "scaling", "rotation", "opacity")
+SKETCH_BUCKETS = 32
+
+
+def sketch(x, seed=7):
+    """Count sketch of a tensor: every entry is added, with a fixed random sign, to one of SKETCH_BUCKETS fixed random
+    buckets.  For a stored reference r and a candidate x, |sketch(x) - sketch(r)| estimates |x - r| (relative spread
+    ~ 1/sqrt(2 * SKETCH_BUCKETS)) from every entry, where storing r itself would take megabytes."""
+    x = np.asarray(x.detach() if isinstance(x, torch.Tensor) else x, np.float64).ravel()
+    rng = np.random.default_rng(seed)
+    bucket = rng.integers(0, SKETCH_BUCKETS, x.size)
+    sign = rng.integers(0, 2, x.size) * 2.0 - 1.0
+    return np.bincount(bucket, weights=sign * x, minlength=SKETCH_BUCKETS)
+
+
+def sketched_rel(x, ref_sketch, ref_norm, seed=7):
+    """Estimate of |x - r| / |r| from r's sketch and norm."""
+    return float(np.linalg.norm(sketch(x, seed) - ref_sketch) / (ref_norm + 1e-30))
 
 
 def reference_dit_case(name):

@@ -1,5 +1,6 @@
-"""GaussianModel post-processing after the sampler loop (SURVEY 8f row 3): filters against the REFERENCE's own GaussianModel
-(gs_core.py:386-475, executed by path) and the PLY export (gs_core.py:577-713) by parsing the written file."""
+"""GaussianModel post-processing after the sampler loop (SURVEY 8f row 3): filters against what the REFERENCE's own
+GaussianModel (gs_core.py:386-475, executed by path in tests/golden/make_renderer_golden.py) kept, and the PLY export
+(gs_core.py:577-713) by parsing the written file."""
 import os
 import sys
 
@@ -9,33 +10,23 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "golden"))
-import ref_import as ri  # noqa: E402
+import make_renderer_golden as mg  # noqa: E402
 
 from dgs_b200.renderer import GaussianModel  # noqa: E402
 
 
-def _data(n=500, seed=0):
-    g = torch.Generator().manual_seed(seed)
-    return (torch.randn(n, 3, generator=g) * 0.8, torch.randn(n, 1, 3, generator=g), torch.randn(n, 3, generator=g) - 3,
-            torch.randn(n, 4, generator=g), torch.randn(n, 1, generator=g) * 2)
-
-
-@pytest.mark.skipif(not ri.available(), reason="/root/reference not mounted")
 def test_filters_equal_reference_gaussian_model():
-    ns = ri.load("oracle")
-    cams = torch.tensor([[0.0, 0.0, 3.0], [3.0, 0.0, 0.0], [0.0, 3.0, 1.0]])
-    ours = GaussianModel(0).set_data(*_data())
-    ref = ns.gs_core.GaussianModel(0).set_data(*_data())
-    ours.apply_all_filters(opacity_thres=0.05, crop_bbx=[-1, 1, -1, 1, -1, 1], cam_origins=cams, nearfar_percent=(0.005, 1.0))
-    ref.apply_all_filters(opacity_thres=0.05, crop_bbx=[-1, 1, -1, 1, -1, 1], cam_origins=cams, nearfar_percent=(0.005, 1.0))
+    ref = np.load(mg.GAUSSIAN_MODEL)
+    ours = GaussianModel(0).set_data(*mg.gaussian_data())
+    ours.apply_all_filters(**mg.FILTERS)
     assert 0 < ours._xyz.shape[0] < 500
-    for k in ("_xyz", "_features_dc", "_scaling", "_rotation", "_opacity"):
-        assert torch.equal(getattr(ours, k), getattr(ref, k)), k
-    assert ours.construct_dtypes() == ref.construct_dtypes()
+    for k in mg.GAUSSIAN_MODEL_FIELDS:
+        assert torch.equal(getattr(ours, k), torch.from_numpy(ref[k])), k
+    assert ours.construct_dtypes() == [tuple(e.split(":")) for e in ref["dtypes"]]
 
 
 def test_save_ply_layout(tmp_path):
-    m = GaussianModel(0).set_data(*_data(37, seed=3))
+    m = GaussianModel(0).set_data(*mg.gaussian_data(37, seed=3))
     path = m.save_ply(str(tmp_path / "sub" / "g.ply"))
     raw = open(path, "rb").read()
     head, body = raw.split(b"end_header\n", 1)

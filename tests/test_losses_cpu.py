@@ -1,72 +1,39 @@
-"""Loss stage (SURVEY 8f row 1) host logic on CPU tensors: dgs_b200.losses.LossComputer / C against the REFERENCE's own
-LossComputer (diffusionGS/utils/losses.py:239-369) and schedule function C (utils/misc.py:73-94), executed by path with
-the absent packages (lpips, pytorch_msssim, skimage) stubbed by deterministic stand-in modules."""
-import importlib.util
+"""Loss stage (SURVEY 8f row 1) host logic on CPU tensors: dgs_b200.losses.LossComputer / C against what the REFERENCE's
+own LossComputer (diffusionGS/utils/losses.py:239-369) returned on the same inputs (tests/golden/make_losses_golden.py,
+the absent packages lpips, pytorch_msssim and skimage stubbed by deterministic stand-in modules), and schedule function C
+(utils/misc.py:73-94)."""
 import os
 import sys
-import types
 
+import numpy as np
 import pytest
 import torch
 import torch.nn as nn
 
 from dgs_b200 import losses
 
-REF = "/root/reference"
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
+import make_losses_golden as mlg  # noqa: E402
 
 
-class _FakeLPIPS(nn.Module):  # stand-in with LPIPS' call signature: per-image scalar [n,1,1,1]
-    def __init__(self, net="vgg"):
-        super().__init__()
-        self.w = nn.Parameter(torch.ones(1))
-
+class _SsimLoss(nn.Module):  # the reference's SsimLoss (losses.py:216-236) around the SSIM stand-in
     def forward(self, x, y):
-        return ((x - y) ** 2).mean(dim=(1, 2, 3), keepdim=True) * self.w
+        return 1 - mlg.FakeSSIM()(x, y)
 
 
-class _FakeSSIM(nn.Module):  # pytorch_msssim.SSIM(size_average=False) -> [n]
-    def __init__(self, **kw):
-        super().__init__()
-
-    def forward(self, x, y):
-        return 1.0 - (x - y).abs().mean(dim=(1, 2, 3))
-
-
-def _load_reference_losses():
-    for name, attrs in (("lpips", dict(LPIPS=_FakeLPIPS)), ("pytorch_msssim", dict(SSIM=_FakeSSIM)),
-                        ("skimage", {}), ("skimage.metrics", dict(structural_similarity=None))):
-        m = types.ModuleType(name)
-        m.__dict__.update(attrs)
-        m.__path__ = []
-        sys.modules.setdefault(name, m)
-    spec = importlib.util.spec_from_file_location("_ref_losses", os.path.join(REF, "diffusionGS/utils/losses.py"))
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod
-
-
-@pytest.mark.skipif(not os.path.isdir(REF), reason="/root/reference not mounted")
-@pytest.mark.parametrize("tc", [3, 4])
+@pytest.mark.parametrize("tc", mlg.TARGET_CHANNELS)
 def test_loss_computer_equals_reference(tc):
-    ref_mod = _load_reference_losses()
-    ref = ref_mod.LossComputer()
-    ours = losses.LossComputer(lpips_module=_FakeLPIPS(), ssim_module=ref.ssim_loss_module, compute_pointsdist=True)
-    g = torch.Generator().manual_seed(0)
-    b, v, h, w = 2, 3, 16, 24
-    rendering = torch.rand(b, v, 3, h, w, generator=g, requires_grad=True)
-    target = torch.rand(b, v, tc, h, w, generator=g)
-    masks = (torch.rand(b, v, 1, h, w, generator=g) > 0.3).float()
-    ray_o = torch.randn(b, v, 3, h, w, generator=g)
-    xyz = torch.randn(b, v, 3, h, w, generator=g, requires_grad=True)
-    gt_xyz = torch.randn(b, v, 3, h, w, generator=g)
-    a = ref(rendering, target, masks, masks, ray_o, img_aligned_xyz=xyz, gt_img_aligned_xyz=gt_xyz)
+    z = np.load(mlg.PATH)
+    a = [torch.from_numpy(z[f"tc{tc}/{k}"]) for k in mlg.TERMS]
+    ours = losses.LossComputer(lpips_module=mlg.FakeLPIPS(), ssim_module=_SsimLoss(), compute_pointsdist=True)
+    rendering, target, masks, ray_o, xyz, gt_xyz = mlg.inputs(tc)
     o = ours(rendering, target, masks, masks, ray_o, img_aligned_xyz=xyz, gt_img_aligned_xyz=gt_xyz)
-    for name, x, y in zip(("l2", "lpips", "ssim", "pointsdist", "l2_xyz"), o, a):
+    for name, x, y in zip(mlg.TERMS, o, a):
         assert x.shape == y.shape, name
         assert torch.allclose(x, y, rtol=1e-6, atol=1e-8), name
     # the l2 handed in from the fused rasterizer path is used verbatim
-    o2 = ours(rendering, target, masks, masks, ray_o, img_aligned_xyz=xyz, gt_img_aligned_xyz=gt_xyz, l2_loss=a[0].detach() * 2)
-    assert torch.equal(o2[0], a[0].detach() * 2)
+    o2 = ours(rendering, target, masks, masks, ray_o, img_aligned_xyz=xyz, gt_img_aligned_xyz=gt_xyz, l2_loss=a[0] * 2)
+    assert torch.equal(o2[0], a[0] * 2)
 
 
 def test_schedule_function_c():

@@ -1,13 +1,14 @@
 """Pins oracle/dit.py (and, on the GPU, the CUDA denoiser itself) to the REFERENCE'S OWN denoiser code.
 
-* live (needs /root/reference, i.e. this container): the reference's DGSDenoiser classes from
-  diffusionGS/models/denoiser/denoiser.py and denoiser_scene.py -- with DiTBlock / modulate from
-  models/transformers/utils_transformer.py -- are executed by path (tests/golden/ref_import.py; only absent third-party
-  packages are stubbed) and oracle/dit.py must equal them to 1e-6 relative, outputs AND parameter gradients;
-* fixtures (any box): tests/golden/dit_ref_*.npz hold what that reference code produced
-  (tests/golden/make_dit_golden.py); the oracle must reproduce them, and on a GPU the product's dgs_dit_forward must
-  match them within the north-star bound for bf16 (1e-3 relative, norm-wise).
+tests/golden/make_dit_golden.py executes the reference's DGSDenoiser classes from diffusionGS/models/denoiser/denoiser.py
+and denoiser_scene.py -- with DiTBlock / modulate from models/transformers/utils_transformer.py -- by path
+(tests/golden/ref_import.py; only absent third-party packages are stubbed) and stores what they produce:
+* tests/golden/dit_ref_pins.npz: the reference's parameter names and shapes, gradient norms and sketches, and the outputs
+  of its building blocks; oracle/dit.py must equal them to 1e-6 relative (outputs) and 2e-5 (parameter gradients);
+* tests/golden/dit_ref_*.npz: the outputs of every case; the oracle must reproduce them, and on a GPU the product's
+  dgs_dit_forward must match them within the north-star bound for bf16 (1e-3 relative, norm-wise).
 """
+import hashlib
 import os
 import sys
 
@@ -17,6 +18,7 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "golden"))
+import make_dit_golden as mdg  # noqa: E402
 import ref_import as ri  # noqa: E402
 
 from oracle.dit import DenoiserOracle  # noqa: E402
@@ -43,45 +45,42 @@ def _fixture(name):
     return {k[4:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("out/")}, z
 
 
-@pytest.mark.skipif(not ri.available(), reason="/root/reference not mounted")
-@pytest.mark.parametrize("name", SMALL + WIDE[:1])
+@pytest.mark.parametrize("name", mdg.PINNED)
 def test_oracle_equals_reference_code(name):
     torch.manual_seed(0)
-    model, (img, ro, rd, t), outs, grads, cot = ri.reference_dit_case(name)
+    _, _, _, (b, v, h, w), seed = ri.DIT_CASES[name]
+    pins = np.load(mdg.PINS)
     o = _oracle_for(name)
-    # identical module tree: the reference's state_dict loads strictly (same keys and shapes)
-    o.load_state_dict(model.state_dict(), strict=True)
+    # identical module tree: the reference's parameters, seeded in its own order, load strictly (same keys and shapes)
+    o.load_state_dict(ri.seeded_params(mdg.shapes(pins, name), seed), strict=True)
+    img, ro, rd, t = ri.seeded_dit_inputs(b, v, h, w, seed + 1000)
     oo, oia = o.image_to_gaussians(img, ro, rd, t)
     oo = dict(oo, img_aligned_xyz=oia)
+    outs, _ = _fixture(name)
     for k in outs:
         e = rel(oo[k].detach(), outs[k])
         assert e < 1e-6, (name, k, e)
+    cot = {k: ri.seeded(tuple(oo[k].shape), seed + 2000 + i) for i, k in enumerate(ri.GS_KEYS)}
     loss = sum((oo[k] * cot[k]).sum() for k in cot)
     og = torch.autograd.grad(loss, list(o.parameters()))
-    worst = max(rel(g, grads[k]) for (k, _), g in zip(o.named_parameters(), og))
+    ref = mdg.gradient_digests(pins, name)
+    worst = max(ri.sketched_rel(g, *ref[k]) for (k, _), g in zip(o.named_parameters(), og))
     assert worst < 2e-5, (name, worst)  # fp32 autograd through SDPA vs explicit softmax: summation order only
 
 
-@pytest.mark.skipif(not ri.available(), reason="/root/reference not mounted")
 def test_reference_blocks_one_by_one():
     """TimestepEmbedder, DiTBlock, GaussiansUpsampler, ImageTokenDecoder of the reference, each against its restatement."""
-    from types import SimpleNamespace
-
     from oracle import dit as od
-    ns = ri.load("stub")
-    torch.manual_seed(3)
-    D, H = 128, 4
-    x, c = torch.randn(2, 37, D), torch.randn(2, D)
-    pairs = [(ns.utils_transformer.DiTBlock(D, H), od.DiTBlock(D, H), (x, c)),
-             (ns.denoiser.TimestepEmbedder(D), od.TimestepEmbedder(D), (torch.tensor([3, 977]),)),
-             (ns.denoiser.GaussiansUpsampler(SimpleNamespace(width=D, gaussians_sh_degree=0)), od._Head(D, 14), (x, c)),
-             (ns.denoiser.ImageTokenDecoder(SimpleNamespace(width=D, gaussians_sh_degree=0, patch_size=4)), od._Head(D, 16 * 14), (x, c))]
-    for ref, mine, args in pairs:
-        sd = ri.seeded_state_dict(ref, 5)
-        ref.load_state_dict(sd, strict=True)
-        mine.load_state_dict(sd, strict=True)
-        assert rel(mine(*args), ref(*args)) < 1e-6, type(ref).__name__
-    assert rel(od.modulate(x, c, 2 * c), ns.utils_transformer.modulate(x, c, 2 * c)) == 0.0
+    pins = np.load(mdg.PINS)
+    D, H = mdg.BLOCK_WIDTH, mdg.BLOCK_HEADS
+    x, c, t = mdg.block_inputs()
+    mine = {"DiTBlock": (od.DiTBlock(D, H), (x, c)), "TimestepEmbedder": (od.TimestepEmbedder(D), (t,)),
+            "GaussiansUpsampler": (od._Head(D, 14), (x, c)), "ImageTokenDecoder": (od._Head(D, 16 * 14), (x, c))}
+    for name, (m, args) in mine.items():
+        m.load_state_dict(ri.seeded_params(mdg.shapes(pins, "blocks/" + name), 5), strict=True)
+        assert rel(m(*args), torch.from_numpy(pins[f"blocks/{name}/out"])) < 1e-6, name
+    # bit-exact: the digest of the reference's modulate() output
+    assert hashlib.sha256(od.modulate(x, c, 2 * c).numpy().tobytes()).hexdigest() == str(pins["blocks/modulate_sha256"])
 
 
 def test_oracle_attention_equals_sdpa():

@@ -1,15 +1,23 @@
 """GPU parity tests of the sm_100a rasterizer, all through the C ABI (libdgs_b200.so):
   * vs the CPU oracle (oracle/raster_oracle.c) on seeded C1 scenes,
-  * vs the UNMODIFIED reference kernels compiled into oracle/_ref (when present),
+  * vs what the UNMODIFIED reference kernels computed on seeded C1 scenes (tests/golden/ref_*.npz, tests/golden/make_golden.py),
   * drop-in package autograd contract, batched renderer, edge cases, full-size properties.
 Tolerance (BASELINE north_star): 1e-4 relative (norm-wise) on colour and on every gradient; integer
 outputs (radii, num_rendered, sorted lists, n_contrib) bit-exact up to the rare fp32 threshold flips
 that FMA contraction differences between compilers can cause (bounded explicitly below)."""
+import json
+import os
+import sys
+
 import numpy as np
 import pytest
 import torch
 
 from util import max_abs, oracle_forward, rel_l2, scene_c1
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+sys.path.insert(0, GOLDEN)
+import make_golden  # noqa: E402
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-4
@@ -62,29 +70,6 @@ def check_grads(ours, ref, tag, skip=(), noise_floor=None):
         assert err < tol, (tag, name, err)
 
 
-def reference_noise_floor(sc, st, dpix, sh, degree, colors=None, cov3d=None):
-    """rel_l2 of the reference kernels' own fp32 gradients vs the oracle (None if oracle/_ref is absent)."""
-    from oracle import build_ref
-    from oracle import raster as orc
-    ref = build_ref.load_module()
-    if ref is None:
-        return None
-    a = sc["act"]
-    e = torch.empty(0, device=DEV)
-    col = e if colors is None else T(colors)
-    cov = e if cov3d is None else T(cov3d)
-    args = (T(np.ones(3)), T(a["means3D"]), col, T(a["opacities"]), e if cov3d is not None else T(a["scales"]),
-            e if cov3d is not None else T(a["rotations"]), 1.0, cov, T(sc["view"]), T(sc["proj"]), float(sc["tanx"]),
-            float(sc["tany"]), sc["H"], sc["W"], e if colors is not None else T(sh), degree, T(sc["campos"]), False,
-            False)
-    Rr, _, radii_r, geom_r, bin_r, img_r = ref.rasterize_gaussians(*args)
-    gr = ref.rasterize_gaussians_backward(args[0], args[1], radii_r, col, args[4], args[5], 1.0, cov, args[8], args[9],
-                                          args[10], args[11], T(dpix), args[14], degree, args[16], geom_r, Rr, bin_r,
-                                          img_r, False)
-    g_or = orc.rasterize_backward(st, dpix)
-    return {n: rel_l2(t.cpu().numpy(), g_or[n]) for n, t in zip(GRAD_NAMES, gr) if g_or[n].size}
-
-
 @pytest.mark.parametrize("dist", ["trained", "init", "fine"])
 def test_c1_forward_backward_vs_oracle(dist):
     from oracle import raster as orc
@@ -116,64 +101,38 @@ def test_c1_forward_backward_vs_oracle(dist):
     check_grads(g, g_ref, dist)
 
 
-@pytest.mark.parametrize("dist", ["trained", "init"])
-def test_c1_vs_reference_kernels(dist):
-    """Three-way agreement: our kernels vs the reference's own kernels (oracle/_ref/dgr_ref_C.so)."""
-    from oracle import build_ref
-    ref = build_ref.load_module()
-    if ref is None:
-        pytest.skip("oracle/_ref/dgr_ref_C.so not built")
-    sc = scene_c1(P=10000, dist=dist)
-    a = sc["act"]
-    e = torch.empty(0, device=DEV)
-    args = (T(np.ones(3)), T(a["means3D"]), e, T(a["opacities"]), T(a["scales"]), T(a["rotations"]), 1.0, e,
-            T(sc["view"]), T(sc["proj"]), float(sc["tanx"]), float(sc["tany"]), sc["H"], sc["W"], T(a["shs"]), 0,
-            T(sc["campos"]), False, False)
-    Rr, color_r, radii_r, geom_r, bin_r, img_r = ref.rasterize_gaussians(*args)
-    fwd = ours_forward(sc)
-    R, color, radii = fwd[0], fwd[1], fwd[2]
-    print(f"[{dist}] R ours={R} ref={Rr}; colour rel_l2={rel_l2(color.cpu().numpy(), color_r.cpu().numpy()):.3e}")
+@pytest.mark.parametrize("case", [c[0] for c in make_golden.CASES])
+def test_c1_vs_reference_kernels(case):
+    """Three-way agreement: our kernels vs the reference's own kernels (oracle/build_ref.py), as they ran on a B200 on the
+    same seeded scene, SH coefficients and dL/dpix (tests/golden/ref_<case>.npz)."""
+    z = np.load(os.path.join(GOLDEN, f"ref_{case}.npz"))
+    sc = scene_c1(P=int(z["P"]), dist=str(z["dist"]), W=int(z["W"]), H=int(z["H"]), seed=int(z["seed"]))
+    deg = int(z["degree"])
+    sh = z["sh"] if deg > 0 else None
+    Rr, radii_r = int(z["num_rendered"]), z["radii"].astype(np.int64)
+    fwd = ours_forward(sc, sh=sh, degree=deg)
+    R, color, radii = fwd[0], fwd[1].cpu().numpy(), fwd[2].cpu().numpy().astype(np.int64)
+    print(f"[{case}] R ours={R} ref={Rr}; colour rel_l2={rel_l2(color, z['color']):.3e}")
     # radius = ceil(3 sqrt(lambda)) may flip by one on an exact-integer boundary (FMA contraction differs between
     # the two compilations); bound it instead of demanding bit equality
     n_bad = int((radii != radii_r).sum())
-    assert n_bad <= 2 and int((radii - radii_r).abs().max()) <= 1 and abs(R - Rr) <= 64, (n_bad, R, Rr)
-    assert rel_l2(color.cpu().numpy(), color_r.cpu().numpy()) < TOL
-    dpix = T(np.random.default_rng(1).normal(0, 1, (3, sc["H"], sc["W"])))
-    gr = ref.rasterize_gaussians_backward(args[0], args[1], radii_r, e, args[4], args[5], 1.0, e, args[8], args[9],
-                                          args[10], args[11], dpix, args[14], 0, args[16], geom_r, Rr, bin_r, img_r,
-                                          False)
-    g = ours_backward(sc, fwd, dpix.cpu().numpy())
-    ref_d = {n: t.cpu().numpy() for n, t in zip(GRAD_NAMES, gr)}
-    check_grads(g, ref_d, "ref-" + dist)
+    assert n_bad <= 2 and int(np.abs(radii - radii_r).max()) <= 1 and abs(R - Rr) <= 64, (n_bad, R, Rr)
+    assert rel_l2(color, z["color"]) < TOL
+    g = ours_backward(sc, fwd, z["dL_dcolor"], sh=sh, degree=deg)
+    check_grads(g, {n: z[n] for n in GRAD_NAMES}, "ref-" + case)
 
 
 def test_sh_degree3_colors_precomp_cov_precomp():
     from oracle import raster as orc
-    sc = scene_c1(P=3000, dist="trained", W=160, H=96)
-    rng = np.random.default_rng(7)
-    dpix = rng.normal(0, 1, (3, sc["H"], sc["W"])).astype(np.float32)
-    sh = rng.normal(0, 0.4, (sc["P"], 16, 3)).astype(np.float32)
-    for deg in (1, 2, 3):
-        st = oracle_forward(sc, sh=sh, degree=deg)
-        fwd = ours_forward(sc, sh=sh, degree=deg)
+    sc, dpix, cases = make_golden.precomp_cases()
+    floors = json.load(open(make_golden.NOISE_FLOORS))  # what the reference kernels measured on these cases
+    for tag, kw in cases.items():
+        st = oracle_forward(sc, **kw)
+        fwd = ours_forward(sc, **kw)
         assert rel_l2(fwd[1].cpu().numpy(), st["color"]) < TOL
-        floor = reference_noise_floor(sc, st, dpix, sh, deg)
-        print(f"  [sh{deg}] reference-kernel noise floor vs oracle: {floor}")
-        check_grads(ours_backward(sc, fwd, dpix, sh=sh, degree=deg), orc.rasterize_backward(st, dpix), f"sh{deg}",
-                    noise_floor=floor)
-    cols = rng.uniform(0, 1, (sc["P"], 3)).astype(np.float32)
-    st = oracle_forward(sc, colors=cols)
-    fwd = ours_forward(sc, colors=cols)
-    assert rel_l2(fwd[1].cpu().numpy(), st["color"]) < TOL
-    check_grads(ours_backward(sc, fwd, dpix, colors=cols), orc.rasterize_backward(st, dpix), "colors_precomp",
-                noise_floor=reference_noise_floor(sc, st, dpix, None, 0, colors=cols))
-    cov = oracle_forward(sc)["cov3D"]
-    st = oracle_forward(sc, cov3d=cov)
-    fwd = ours_forward(sc, cov3d=cov)
-    assert rel_l2(fwd[1].cpu().numpy(), st["color"]) < TOL
-    check_grads(ours_backward(sc, fwd, dpix, cov3d=cov), orc.rasterize_backward(st, dpix), "cov_precomp",
-                skip=("dL_dscales", "dL_drotations"),
-                noise_floor=reference_noise_floor(sc, st, dpix, sc["act"]["shs"], 0, cov3d=cov))
+        print(f"  [{tag}] reference-kernel noise floor vs oracle: {floors[tag]}")
+        check_grads(ours_backward(sc, fwd, dpix, **kw), orc.rasterize_backward(st, dpix), tag,
+                    skip=("dL_dscales", "dL_drotations") if "cov3d" in kw else (), noise_floor=floors[tag])
 
 
 def test_edge_cases_empty_culled_ragged():
